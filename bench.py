@@ -11,7 +11,7 @@ beside the step for the per-iteration roofline of the SpMV/PCG kernels)
 `parts` carries the other two components (DP return map Mpts/s, PCG-Newton s/step with ms/iteration) and
 `rooflines` the achieved HBM bandwidth of every kernel against MEASURED_PEAKS.json.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--nx 2828] [--pcg-iters 20]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--nx 2828] [--pcg-iters 20] [--dump-outputs DIR]
     python bench.py --impl reference      # the oracle port of the reference's CPU path on a bounded sample
 """
 import argparse
@@ -303,6 +303,26 @@ def bind_to_gpu_numa_node(index):
     return "not bound"
 
 
+DUMP_SAMPLE = 1 << 18   # entries kept along the last axis of an output: at most 41 MB for all outputs of a step
+
+
+def dump_outputs(out_dir, arrays, rank, world):
+    """Writes each tensor as out_dir/<name>.npy (<name>_rank<r>.npy when several ranks run).  Along its last axis an array
+    longer than DUMP_SAMPLE / world keeps the entries at a fixed seeded sample of indices, the same in every run of the same
+    size, so that the outputs of two builds can be compared entry for entry.  Integer outputs are written as floats."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    cap = DUMP_SAMPLE // world
+    for name, t in arrays.items():
+        n = t.shape[-1]
+        if n > cap:
+            idx = np.sort(np.random.default_rng(0).choice(n, cap, replace=False))
+            t = t.index_select(t.dim() - 1, torch.as_tensor(idx, device=t.device))
+        a = t.cpu().numpy()
+        a = a.astype(np.float64 if a.dtype.itemsize == 8 else np.float32)      # int64 counts are exact in float64
+        np.save(os.path.join(out_dir, name + (f"_rank{rank}" if world > 1 else "") + ".npy"), a)
+
+
 # ------------------------------------------------------------------------------------------------
 # GPU side
 # ------------------------------------------------------------------------------------------------
@@ -366,7 +386,7 @@ def run_gpu(args):
         except Exception as e:  # noqa: BLE001  (e.g. no symmetric memory on this box: every rank fails at the same collective)
             mgs, solver_note = None, f"multigrid unavailable ({type(e).__name__}: {e}); step timed with {args.pcg_iters} fixed Jacobi-PCG iterations"
             print(solver_note, file=sys.stderr)
-    solve_info = {}
+    solve_info, last = {}, {}
 
     def ev():
         return torch.cuda.Event(enable_timing=True)
@@ -392,7 +412,7 @@ def run_gpu(args):
             x, its = pcg.solve(k_tan, rhs, iters=args.pcg_iters)
             n_launch = pcg.launches_last
         evs[4].record()
-        pcg.energy_norms(k_el, x, u, rhs)
+        last["solution"], last["energy_norms"] = x, pcg.energy_norms(k_el, x, u, rhs)
         evs[5].record()
         launches["n"] = 1 + 1 + 1 + 1 + n_launch + 3
         if record is not None:
@@ -422,6 +442,10 @@ def run_gpu(args):
     clocks = sampler.stop() if rank == 0 else None
     total_ms = t0.elapsed_time(t1)
     per = {p: float(np.mean([e[i].elapsed_time(e[i + 1]) for e in rec])) for i, p in enumerate(phases)}
+    if args.dump_outputs:                                # before anything below overwrites the step's buffers
+        dump_outputs(args.dump_outputs, {"strain": E, "stress": rm["s"], "tangent_operator": rm["ds"], "plastic": rm["ind_p"],
+                                         "plastic_counts": rm["counts"], "k_tangent": k_tan, "internal_force": F, **last},
+                     rank, world)
     # ---- isolated kernels (same inputs, outside the step): K_tangent alone and K_elast
     def iso(fn, reps=5):
         fn()
@@ -714,7 +738,13 @@ def main():
     ap.add_argument("--no-strong", action="store_true", help="skip the strong-scaling part of an N > 1 run")
     ap.add_argument("--halo", default="auto", choices=["auto", "nccl", "peer", "fused"], help="multi-GPU exchanges of the PCG: fused = inside the kernels over NVLink peer memory; auto = fused, NCCL if symmetric memory is unavailable")
     ap.add_argument("--no-graph", action="store_true", help="launch the PCG iterations eagerly instead of replaying a CUDA graph")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the arrays the last one computed as DIR/<name>.npy "
+                                                           "(float64, or float32 for flags; a fixed sample of each larger array, 41 MB at most)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl b200)")
     if args.impl == "reference":
         run_reference(args)
     else:
