@@ -75,6 +75,9 @@ SIGNATURES = {
     "fem_peer_allreduce": [_vp, _i32, _vp, C.POINTER(_vp), _i64, _i64, _i64, _i32, _i32, _vp],
     "fem_mg_fine_step": [_vp, _vp, _i32, _vp, _vp, _vp, _vp, _dbl, _dbl, _vp, _vp],
     "fem_mg_to_f32": [_i64, _vp, _vp, _vp],
+    "fem_mg_lattice_check": [_vp, _vp, _i32, _vp, _vp],
+    "fem_mg_to_f32_lattice": [_vp, _vp, _vp, _vp, _i64, _i32, _i32, _vp],
+    "fem_mg_fine_step_lattice": [_vp, _vp, _i32, _vp, _vp, _vp, _dbl, _dbl, _vp, _vp],
     "fem_mg_exchange_run": [_vp, _vp, _vp, _vp],
     "fem_mg_pcg_init": [_i64, _vp, _vp, _vp, _vp, _vp, _vp],
     "fem_mg_pcg_update_xr": [_i64, _vp, _vp, _vp, _vp, _vp, _i32, _vp],

@@ -38,6 +38,7 @@ struct FemTuning {
   int assemble_canon;      // 0 auto (straight-line path for slices of the reference's regular triangulation), 2 off
   int strain_variant;      // 0/1 stored gradients (default), 2 P1 gradients recomputed from the coordinates (slower: L2 gathers)
   int mg_stencil_sym;      // 0 auto: coarse-level stencil sweeps read the lower half of the (symmetric) stencil as transposes of the neighbours' upper half; 2 = read all 36 planes
+  int mg_fine_lattice;     // 0 auto: the V-cycle's level-0 smoother and residual read the lattice stencil when the descriptor carries one; 2 = the block-CSR copy
   int peer_nowait;         // DIAGNOSTIC ONLY: fused multi-GPU PCG kernels skip their waits (wrong results; isolates the wait time)
 };
 extern FemTuning g_fem_tuning;

@@ -770,6 +770,172 @@ __global__ void __launch_bounds__(256) mg_to_f32_kernel(int64_t n4, const double
   }
 }
 
+// ---- level 0 on the lattice: the smoother and the residual as a symmetric FP32 stencil ---------------------------------
+// When node id == lattice point (iy * LX + ix) and the triangulation has one diagonal orientation, every node couples to
+// E, W, N, S and one diagonal pair (NE + SW or NW + SE): a 7-point stencil of 2x2 blocks.  The matrix is symmetric, so
+// only the upper half is stored - the self block and the blocks towards E, N and the upper diagonal neighbour, 16 planes
+// of FP32 = 64 B per node and no index bytes (the block-CSR copy: 112 B of values + 14 B of block positions + the row
+// pointers).  The blocks towards W, S and the lower diagonal neighbour are the transposes of those neighbours' E, N and
+// diagonal blocks.
+enum { LAT_SELF = 0, LAT_E = 1, LAT_N = 2, LAT_D = 3 };
+
+__global__ void __launch_bounds__(256) mg_lattice_check_kernel(int64_t n_n, const int32_t* __restrict__ nbr_ptr, const int32_t* __restrict__ nbr_idx,
+                                                               const int32_t* __restrict__ node_lat, int LX, int32_t* err) {
+  for (int64_t a = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; a < n_n; a += (int64_t)gridDim.x * blockDim.x) {
+    int e = node_lat[a] != (int32_t)a ? 1 : 0;
+    const int64_t ia = a % LX, ja = a / LX;
+    for (int p = nbr_ptr[a]; p < nbr_ptr[a + 1]; ++p) {
+      const int64_t b = nbr_idx[p];
+      const int64_t dx = b % LX - ia, dy = b / LX - ja;
+      if (dx < -1 || dx > 1 || dy < -1 || dy > 1) e |= 2;
+      else if (dx * dy == 1) e |= 4;
+      else if (dx * dy == -1) e |= 8;
+    }
+    if (e) atomicOr(err, e);
+  }
+}
+
+// one thread per node: its block-CSR row of FP64 values -> the FP32 copy of the row (the layout fem_mg_to_f32 writes) and
+// its four upper-half blocks -> the planes (zero where the neighbour does not exist).  Plain FP32 rounding of the same values.
+__global__ void __launch_bounds__(256) mg_to_f32_lattice_kernel(int64_t n_n, const int32_t* __restrict__ nbr_ptr, const int32_t* __restrict__ nbr_idx,
+                                                                const double* __restrict__ vals, float* __restrict__ k32, float* __restrict__ planes,
+                                                                int64_t stride, int LX, int64_t diag_off) {
+  for (int64_t a = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; a < n_n; a += (int64_t)gridDim.x * blockDim.x) {
+    const int p0 = nbr_ptr[a], deg = nbr_ptr[a + 1] - p0;
+    const double2* r0 = reinterpret_cast<const double2*>(vals + 4 * (int64_t)p0);
+    const double2* r1 = r0 + deg;
+    float2* o0 = reinterpret_cast<float2*>(k32 + 4 * (int64_t)p0);
+    float2* o1 = o0 + deg;
+    float s[16];
+#pragma unroll
+    for (int q = 0; q < 16; ++q) s[q] = 0.0f;
+    for (int j = 0; j < deg; ++j) {
+      const double2 u = __ldcs(r0 + j), v = __ldcs(r1 + j);
+      const float2 fu = make_float2((float)u.x, (float)u.y), fv = make_float2((float)v.x, (float)v.y);
+      o0[j] = fu;
+      o1[j] = fv;
+      const int64_t off = (int64_t)nbr_idx[p0 + j] - a;
+      const int slot = off == 0 ? LAT_SELF : (off == 1 ? LAT_E : (off == LX ? LAT_N : (off == diag_off ? LAT_D : -1)));
+#pragma unroll
+      for (int sl = 0; sl < 4; ++sl)
+        if (slot == sl) {
+          s[4 * sl + 0] = fu.x;
+          s[4 * sl + 1] = fu.y;
+          s[4 * sl + 2] = fv.x;
+          s[4 * sl + 3] = fv.y;
+        }
+    }
+#pragma unroll
+    for (int q = 0; q < 16; ++q) __stcs(planes + q * stride + a, s[q]);
+  }
+}
+
+// One step of the V-cycle's level 0 on the planes, one thread per owned node, nodes in order (the grid walks the lattice
+// row by row): the self block is read once (streaming loads), the E, N and diagonal blocks with cached loads - the E block
+// of node a - 1 comes from the neighbouring lane, the N and diagonal blocks of the row below were read by the blocks just
+// before (L2).  Epilogue: MgStreamEpilogue, the formulas of the block-CSR path (b, D^-1, d, x; Dirichlet mask of the residual).
+template <int MODE, bool NW>
+__global__ void __launch_bounds__(256) mg_fine_lattice_kernel(const float* __restrict__ S, int64_t stride, int LX, int lat_rows, const double* x,
+                                                              const MgStreamEpilogue<MODE> epi, double* dot_out, const FemRedBuf rb) {
+  __shared__ double red[32];
+  const double2* xv = reinterpret_cast<const double2*>(x);
+  const int lane = threadIdx.x & 31;
+  double dot = 0.0;
+  // warp-uniform loop: every lane takes part in the shuffle of the E blocks
+  for (int64_t base = epi.own_lo + (int64_t)blockIdx.x * blockDim.x + (threadIdx.x & ~31); base < epi.own_hi; base += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t a = base + lane;
+    const bool act = a < epi.own_hi;
+    const int64_t ac = act ? a : epi.own_lo;
+    const int i = (int)(ac % LX), j = (int)(ac / LX);
+    const bool hw = i > 0, he = i < LX - 1, hs = j > 0, hn = j < lat_rows - 1;
+    const bool hdu = NW ? (hn && hw) : (hn && he), hdl = NW ? (hs && he) : (hs && hw);
+    const int64_t up_d = NW ? ac + LX - 1 : ac + LX + 1, lo_d = NW ? ac - LX + 1 : ac - LX - 1;
+    float k[4], e[4], nn[4], dd[4], w[4], sb[4], db[4];
+#pragma unroll
+    for (int q = 0; q < 4; ++q) {
+      k[q] = __ldcs(S + (4 * LAT_SELF + q) * stride + ac);
+      e[q] = __ldg(S + (4 * LAT_E + q) * stride + ac);
+      nn[q] = __ldg(S + (4 * LAT_N + q) * stride + ac);
+      dd[q] = __ldg(S + (4 * LAT_D + q) * stride + ac);
+    }
+#pragma unroll
+    for (int q = 0; q < 4; ++q) {
+      w[q] = __shfl_up_sync(0xffffffffu, e[q], 1);
+      if (lane == 0) w[q] = hw ? __ldg(S + (4 * LAT_E + q) * stride + ac - 1) : 0.0f;
+      if (!hw) w[q] = 0.0f;
+      sb[q] = hs ? __ldg(S + (4 * LAT_N + q) * stride + ac - LX) : 0.0f;
+      db[q] = hdl ? __ldg(S + (4 * LAT_D + q) * stride + lo_d) : 0.0f;
+    }
+    const double2 z2 = make_double2(0.0, 0.0);
+    const double2 x0 = xv[ac], xe = he ? xv[ac + 1] : z2, xw = hw ? xv[ac - 1] : z2, xn = hn ? xv[ac + LX] : z2, xs = hs ? xv[ac - LX] : z2;
+    const double2 xdu = hdu ? xv[up_d] : z2, xdl = hdl ? xv[lo_d] : z2;
+    // upper blocks as stored (row i of the block times x of the neighbour), lower blocks transposed
+    double y0 = (double)k[0] * x0.x;
+    y0 = fma((double)k[1], x0.y, y0);
+    double y1 = (double)k[2] * x0.x;
+    y1 = fma((double)k[3], x0.y, y1);
+#define LAT_UP(B, X)                        \
+  y0 = fma((double)B[0], X.x, y0);          \
+  y0 = fma((double)B[1], X.y, y0);          \
+  y1 = fma((double)B[2], X.x, y1);          \
+  y1 = fma((double)B[3], X.y, y1);
+#define LAT_LO(B, X)                        \
+  y0 = fma((double)B[0], X.x, y0);          \
+  y0 = fma((double)B[2], X.y, y0);          \
+  y1 = fma((double)B[1], X.x, y1);          \
+  y1 = fma((double)B[3], X.y, y1);
+    LAT_UP(e, xe)
+    LAT_UP(nn, xn)
+    LAT_UP(dd, xdu)
+    LAT_LO(w, xw)
+    LAT_LO(sb, xs)
+    LAT_LO(db, xdl)
+#undef LAT_UP
+#undef LAT_LO
+    if (act) {
+      double2 sv[MgStreamEpilogue<MODE>::N_IN];
+      uchar2 mk = make_uchar2(1, 1);
+      sv[0] = epi.b[a];
+      if constexpr (MODE == MG_RESID) {
+        if (epi.mask) mk = reinterpret_cast<const uchar2*>(epi.mask)[a];
+      } else {
+        sv[1] = epi.dinv[a];
+        sv[2] = epi.dinv[epi.n_n + a];
+        sv[3] = epi.c1 != 0.0 ? epi.d[a] : z2;  // d is not read when c1 == 0 (first step of a sweep)
+        sv[4] = x0;
+      }
+      epi(a, y0, y1, sv, mk, dot);
+    }
+  }
+  if (dot_out) {
+    const double v[1] = {block_sum(dot, red)};
+    double* const dst[1] = {dot_out};
+    ordered_accumulate<1>(v, dst, rb);
+  }
+}
+
+template <int MODE>
+int launch_fine_lattice(const fem_plan* P, const fem_mg_desc* D, const double* b, const double* x, double* out, double c1, double c2, double* dot,
+                        cudaStream_t st) {
+  const MgStreamEpilogue<MODE> se{reinterpret_cast<const double2*>(b), reinterpret_cast<const double2*>(D->dinv), reinterpret_cast<double2*>(D->d),
+                                  reinterpret_cast<const double2*>(x), reinterpret_cast<double2*>(out), D->mask, c1, c2, dot != nullptr,
+                                  D->own_node_lo, D->own_node_hi, P->n_n};
+  const FemRedBuf rb{P->red_partials, P->red_ticket};
+  const unsigned blocks = vgrid(D->own_node_hi - D->own_node_lo, P->sm_count);  // <= 8 per SM: the ordered dot's slots
+  if (D->lat32_nw) mg_fine_lattice_kernel<MODE, true><<<blocks, 256, 0, st>>>(D->lat32, D->lat32_stride, D->LX, D->lat_rows, x, se, dot, rb);
+  else mg_fine_lattice_kernel<MODE, false><<<blocks, 256, 0, st>>>(D->lat32, D->lat32_stride, D->LX, D->lat_rows, x, se, dot, rb);
+  FEM_CUDA_CHECK(cudaGetLastError());
+  return FEM_OK;
+}
+
+// the V-cycle's level-0 smoother and residual: the lattice stencil when the descriptor carries one, else the block-CSR copy
+template <int MODE>
+int launch_vcycle_fine(const fem_plan* P, const fem_mg_desc* D, const double* K, const double* b, const double* x, double* out, double c1, double c2,
+                       double* dot, cudaStream_t st) {
+  if (D->lat32 && g_fem_tuning.mg_fine_lattice != 2) return launch_fine_lattice<MODE>(P, D, b, x, out, c1, c2, dot, st);
+  return launch_fine<MODE>(P, D, K, b, x, out, c1, c2, dot, st);
+}
+
 #define MG_TRY(expr)             \
   do {                           \
     const int _rc = (expr);      \
@@ -914,6 +1080,25 @@ extern "C" int fem_mg_to_f32(int64_t n, const double* src, float* dst, fem_strea
   return FEM_OK;
 }
 
+extern "C" int fem_mg_lattice_check(const fem_plan* P, const int32_t* node_lat, int LX, int32_t* err, fem_stream stream) {
+  FEM_REQUIRE(P && node_lat && err && LX > 0, "null pointer");
+  cudaStream_t st = (cudaStream_t)stream;
+  mg_lattice_check_kernel<<<vgrid(P->n_n, P->sm_count), 256, 0, st>>>(P->n_n, P->nbr_ptr, P->nbr_idx, node_lat, LX, err);
+  FEM_CUDA_CHECK(cudaGetLastError());
+  return FEM_OK;
+}
+
+extern "C" int fem_mg_to_f32_lattice(const fem_plan* P, const double* K_vals, float* k32, float* planes, int64_t stride, int LX, int nw,
+                                     fem_stream stream) {
+  FEM_REQUIRE(P && K_vals && k32 && planes && stride >= P->n_n && LX > 0, "null pointer or plane stride");
+  FEM_REQUIRE(((reinterpret_cast<uintptr_t>(K_vals) | reinterpret_cast<uintptr_t>(k32)) & 15u) == 0, "16-byte alignment");
+  cudaStream_t st = (cudaStream_t)stream;
+  mg_to_f32_lattice_kernel<<<vgrid(P->n_n, P->sm_count), 256, 0, st>>>(P->n_n, P->nbr_ptr, P->nbr_idx, K_vals, k32, planes, stride, LX,
+                                                                      nw ? (int64_t)LX - 1 : (int64_t)LX + 1);
+  FEM_CUDA_CHECK(cudaGetLastError());
+  return FEM_OK;
+}
+
 extern "C" int fem_mg_exchange_run(const fem_mg_exchange* ex, double* v, uint64_t* err, fem_stream stream) {
   FEM_REQUIRE(ex && v, "null pointer");
   return run_exchange(*ex, v, err, (cudaStream_t)stream);
@@ -950,11 +1135,11 @@ extern "C" int fem_mg_vcycle(const fem_plan* P, const fem_mg_desc* D, const doub
   FEM_CUDA_CHECK(cudaGetLastError());
   for (int s = 1; s < k; ++s) {
     MG_TRY(run_exchange(*ecur, cur, D->err, st));
-    MG_TRY(launch_fine<MG_CHEB>(P, D, K_vals, r, cur, oth, D->c1[s], D->c2[s], nullptr, st));
+    MG_TRY(launch_vcycle_fine<MG_CHEB>(P, D, K_vals, r, cur, oth, D->c1[s], D->c2[s], nullptr, st));
     swap();
   }
   MG_TRY(run_exchange(*ecur, cur, D->err, st));
-  MG_TRY(launch_fine<MG_RESID>(P, D, K_vals, r, cur, D->r, 0.0, 0.0, nullptr, st));
+  MG_TRY(launch_vcycle_fine<MG_RESID>(P, D, K_vals, r, cur, D->r, 0.0, 0.0, nullptr, st));
   MG_TRY(run_exchange(D->ex_r, D->r, D->err, st));
   const fem_mg_level& C = D->lev[0];
   {
@@ -976,7 +1161,7 @@ extern "C" int fem_mg_vcycle(const fem_plan* P, const fem_mg_desc* D, const doub
   for (int s = 0; s < k; ++s) {
     const bool last = s == k - 1;
     MG_TRY(run_exchange(*ecur, cur, D->err, st));
-    MG_TRY(launch_fine<MG_CHEB>(P, D, K_vals, r, cur, last ? z : oth, s == 0 ? 0.0 : D->c1[s], D->c2[s], last ? dot : nullptr, st));
+    MG_TRY(launch_vcycle_fine<MG_CHEB>(P, D, K_vals, r, cur, last ? z : oth, s == 0 ? 0.0 : D->c1[s], D->c2[s], last ? dot : nullptr, st));
     swap();
   }
   return FEM_OK;
@@ -990,6 +1175,14 @@ extern "C" int fem_mg_fine_step(const fem_plan* P, const fem_mg_desc* D, int mod
   cudaStream_t st = (cudaStream_t)stream;
   if (mode == MG_RESID) return launch_fine<MG_RESID>(P, D, K_vals, b, x, out, 0.0, 0.0, nullptr, st);
   return launch_fine<MG_CHEB>(P, D, K_vals, b, x, out, c1, c2, dot, st);
+}
+
+extern "C" int fem_mg_fine_step_lattice(const fem_plan* P, const fem_mg_desc* D, int mode, const double* b, const double* x, double* out,
+                                        double c1, double c2, double* dot, fem_stream stream) {
+  FEM_REQUIRE(P && D && D->lat32 && b && x && out && (mode == MG_RESID || mode == MG_CHEB) && out != x, "arguments");
+  cudaStream_t st = (cudaStream_t)stream;
+  if (mode == MG_RESID) return launch_fine_lattice<MG_RESID>(P, D, b, x, out, 0.0, 0.0, nullptr, st);
+  return launch_fine_lattice<MG_CHEB>(P, D, b, x, out, c1, c2, dot, st);
 }
 
 extern "C" int fem_mg_pcg_init(int64_t n, const double* rhs, const uint8_t* mask, double* r, double* x, double* scal, fem_stream stream) {

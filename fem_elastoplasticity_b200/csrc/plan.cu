@@ -34,6 +34,7 @@ extern "C" int fem_set_tuning(const char* key, int value) {
   else if (!strcmp(key, "strain_variant")) g_fem_tuning.strain_variant = value;
   else if (!strcmp(key, "assemble_canon")) g_fem_tuning.assemble_canon = value;
   else if (!strcmp(key, "mg_stencil_sym")) g_fem_tuning.mg_stencil_sym = value;
+  else if (!strcmp(key, "mg_fine_lattice")) g_fem_tuning.mg_fine_lattice = value;
   else {
     fem_set_error("unknown tuning key %s", key);
     return FEM_ERR_INVALID_ARG;

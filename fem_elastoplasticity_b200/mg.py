@@ -46,7 +46,8 @@ class Desc(C.Structure):
                 ("own_node_hi", C.c_int64), ("mask", C.c_void_p), ("dinv", C.c_void_p), ("xa", C.c_void_p), ("xb", C.c_void_p),
                 ("d", C.c_void_p), ("r", C.c_void_p), ("c1", C.c_double * MAX_DEGREE), ("c2", C.c_double * MAX_DEGREE),
                 ("ex_xa", Exchange), ("ex_xb", Exchange), ("ex_r", Exchange), ("lev", Level * MAX_LEVELS), ("coarse_inv", C.c_void_p),
-                ("K32", C.c_void_p), ("err", C.c_void_p)]
+                ("K32", C.c_void_p), ("err", C.c_void_p), ("lat32", C.c_void_p), ("lat32_stride", C.c_int64), ("lat32_nw", C.c_int32),
+                ("lat32_pad", C.c_int32)]
 
 
 def chebyshev_coefficients(lmax, ratio, degree):
@@ -187,6 +188,7 @@ class MultigridPCG:
             if not bool((self.node_lat == torch.arange(plan.n_n, dtype=torch.int32, device=dev)).all()):
                 raise MultigridUnsupported("partitioned multigrid needs lattice-ordered node numbering")
         self.own_nodes = (own_rows[0] * LX, own_rows[1] * LX) if self.part is not None else (0, plan.n_n)
+        self._lattice_stencil(LX, lat_rows)
         self.layouts = level_layouts(LX, NY, owned, max_coarse_dofs=max_coarse_dofs, replicate_below=replicate_below)
         self.n_levels = len(self.layouts)
         # ---- buffers (on a partition the vectors whose ghost rows travel live in one symmetric-memory arena)
@@ -210,6 +212,36 @@ class MultigridPCG:
         self.coarse_inv, self.desc, self.setup_seconds, self.lmax0 = None, None, None, None
         self._graph, self._graph_key = None, None
         self.launches_last = 0
+
+    def _lattice_stencil(self, LX, lat_rows):
+        """Level 0 as a 7-point stencil (fem_mg_fine_lattice): the FP32 smoother on one GPU, node id == lattice point, every
+        neighbour inside the 3x3 window and one diagonal orientation.  Otherwise (and on strip partitions, where the stencil
+        has not been checked against the ghost rows) the smoother keeps the block-CSR copy."""
+        self.k32s, self.lat32_stride, self.lat32_nw = None, 0, 0
+        P = self.plan
+        if self.k32 is None or self.part is not None or LX * lat_rows != P.n_n:
+            return
+        err = torch.zeros(1, dtype=torch.int32, device=self.device)
+        call("fem_mg_lattice_check", P._h, _ptr(self.node_lat), LX, _ptr(err), _stream())
+        e = int(err.item())
+        if e & 3 or e == 12:
+            return
+        self.lat32_nw = 1 if e == 8 else 0
+        self.lat32_stride = (P.n_n + 31) // 32 * 32                # every plane starts on a 128-byte line
+        self.k32s = torch.zeros(16 * self.lat32_stride, dtype=torch.float32, device=self.device)
+
+    @property
+    def fine_lattice(self):
+        return self.k32s is not None
+
+    def to_f32(self, k_vals):
+        """The FP32 copies the level-0 smoother reads: the block-CSR copy k32 and, when level 0 runs on the lattice, the
+        stencil planes k32s (one pass over k_vals)."""
+        if self.k32s is not None:
+            call("fem_mg_to_f32_lattice", self.plan._h, _ptr(k_vals), _ptr(self.k32), _ptr(self.k32s), self.lat32_stride, self.lattice[4],
+                 self.lat32_nw, _stream())
+        elif self.k32 is not None:
+            call("fem_mg_to_f32", self.plan.nnz, _ptr(k_vals), _ptr(self.k32), _stream())
 
     # -- multi-GPU plumbing (set-up collectives through torch.distributed; the solve uses fem_mg_exchange) ----------------
     def _vec(self, name, size):
@@ -481,6 +513,8 @@ class MultigridPCG:
         d.coarse_inv = self.coarse_inv.data_ptr()
         d.K32 = self.k32.data_ptr() if self.k32 is not None else 0
         d.err = 0
+        if self.k32s is not None:
+            d.lat32, d.lat32_stride, d.lat32_nw = self.k32s.data_ptr(), self.lat32_stride, self.lat32_nw
         self._fill_exchanges(d)
         self.desc = d
 
@@ -509,6 +543,14 @@ class MultigridPCG:
         c1 = self.desc.c1[step] if mode == 2 else 0.0
         c2 = self.desc.c2[step] if mode == 2 else 0.0
         call("fem_mg_fine_step", self.plan._h, C.byref(self.desc), mode, _ptr(k_vals), _ptr(b), _ptr(x), _ptr(out), c1, c2, _ptr(dot), _stream())
+
+    def fine_step_lattice(self, b, x, out, mode=2, step=1, dot=None):
+        """``fine_step`` on the lattice stencil k32s (filled by ``to_f32``) instead of the block-CSR matrix."""
+        if self.k32s is None:
+            raise ValueError("level 0 of this multigrid does not run on the lattice stencil")
+        c1 = self.desc.c1[step] if mode == 2 else 0.0
+        c2 = self.desc.c2[step] if mode == 2 else 0.0
+        call("fem_mg_fine_step_lattice", self.plan._h, C.byref(self.desc), mode, _ptr(b), _ptr(x), _ptr(out), c1, c2, _ptr(dot), _stream())
 
     def _exchange_p(self):
         if self.part is not None:
@@ -555,8 +597,7 @@ class MultigridPCG:
             self.setup(k_vals)
         P, s, n = self.plan, self.scal, self.plan.n_dof
         self.block_jacobi(k_vals)
-        if self.k32 is not None:
-            call("fem_mg_to_f32", P.nnz, _ptr(k_vals), _ptr(self.k32), _stream())
+        self.to_f32(k_vals)
         call("fem_mg_pcg_init", n, _ptr(rhs), _ptr(self.mask), _ptr(self.r), _ptr(self.x), _ptr(s), _stream())
         self._sum_scal(0, 5)
         self.vcycle(k_vals, self.r, self.z, s[0:1])

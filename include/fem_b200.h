@@ -256,6 +256,13 @@ typedef struct fem_mg_desc {
   const float* K32;                  /* optional FP32 copy of K_vals (fem_mg_to_f32): streamed by the level-0 smoother and residual
                                         instead of the FP64 values (half the bytes; sums stay FP64); NULL = use K_vals */
   uint64_t* err;                     /* sticky word: a wait timed out (NULL on one GPU) */
+  const float* lat32;                /* optional level-0 stencil (fem_mg_to_f32_lattice): node id == lattice point, 7-point pattern;
+                                        [16][lat32_stride] planes 4*slot + 2*i + j, slots self, E, N, diagonal (upper half of the
+                                        symmetric matrix).  Read by the V-cycle's level-0 smoother and residual instead of K32
+                                        (NULL: block-CSR path) */
+  int64_t lat32_stride;              /* plane stride (>= n_n, multiple of 32) */
+  int32_t lat32_nw;                  /* diagonal slot: 1 = north-west (the lower partner is south-east), 0 = north-east */
+  int32_t lat32_pad;
 } fem_mg_desc;
 int fem_mg_sizeof(int which); /* sizeof fem_mg_exchange (0), fem_mg_level (1), fem_mg_desc (2): checked by the binding */
 /* set-up steps (once per mesh / per matrix the hierarchy is built from) */
@@ -286,6 +293,15 @@ int fem_peer_allreduce(double* vals, int n, void* comm, const void* const* peers
 int fem_mg_fine_step(const fem_plan* plan, const fem_mg_desc* desc, int mode, const double* K_vals, const double* b, const double* x,
                      double* out, double c1, double c2, double* dot, fem_stream stream);
 int fem_mg_to_f32(int64_t n, const double* src, float* dst, fem_stream stream); /* n % 4 == 0 (nnz of the 2x2-block pattern) */
+/* level-0 stencil on the lattice.  _check (set-up, once per mesh): err |= 1 node id != lattice point, 2 a neighbour outside
+ * the 3x3 window, 4 a north-east/south-west edge, 8 a north-west/south-east edge (the stencil needs err in {0, 4, 8}).
+ * _to_f32_lattice (per matrix): one pass over K_vals writes the FP32 block-CSR copy k32 (== fem_mg_to_f32) and the planes of
+ * fem_mg_desc.lat32.  _fine_step_lattice: fem_mg_fine_step on desc->lat32 (benchmarks, tests).                       */
+int fem_mg_lattice_check(const fem_plan* plan, const int32_t* node_lat, int LX, int32_t* err, fem_stream stream);
+int fem_mg_to_f32_lattice(const fem_plan* plan, const double* K_vals, float* k32, float* planes, int64_t stride, int LX, int nw,
+                          fem_stream stream);
+int fem_mg_fine_step_lattice(const fem_plan* plan, const fem_mg_desc* desc, int mode, const double* b, const double* x, double* out,
+                             double c1, double c2, double* dot, fem_stream stream);
 int fem_mg_exchange_run(const fem_mg_exchange* ex, double* v, uint64_t* err, fem_stream stream);
 /* CG steps around the V-cycle (scal as in fem_pcg_*: [0]/[2] r'z by iteration parity, [1] r'r, [3] p'Kp, [4] |b|^2):
  * init: r = mask .* rhs, x = 0, scal zeroed, [1] = [4] = |r|^2;  update_xr: x += alpha p, r -= alpha q, [1] += r'r;
@@ -333,7 +349,8 @@ int fem_midpoints_p2_fill(void* handle, const double* coord, double* coord_mid, 
 int fem_midpoints_p2_destroy(void* handle, fem_stream stream);
 
 /* launch-shape knobs for benchmarking ("return_map_variant", "assemble_variant", "assemble_warps", "spmv_group", "spmv_blocks_per_sm",
- * "spmv_staged", "peer_timeout_ms", "strain_variant", "assemble_canon");
+ * "spmv_staged", "peer_timeout_ms", "strain_variant", "assemble_canon", "mg_stencil_sym", "mg_fine_lattice" (2: the V-cycle's
+ * level 0 reads the block-CSR copy even when the descriptor carries the lattice stencil));
  * value 0 restores the default.  Results never depend on them.                                     */
 int fem_set_tuning(const char* key, int value);
 
