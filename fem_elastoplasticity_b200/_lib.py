@@ -114,7 +114,7 @@ def load():
     for kv in filter(None, os.environ.get("FEM_B200_TUNING", "").split(",")):      # launch-shape / diagnostic knobs: "key=value,..."
         k, v = kv.split("=")
         if lib.fem_set_tuning(k.strip().encode(), int(v)) != 0:
-            raise ValueError(f"FEM_B200_TUNING: unknown key {k!r}")
+            raise ValueError(f"FEM_B200_TUNING: {kv!r} rejected: {lib.fem_last_error_string().decode()}")
     return lib
 
 

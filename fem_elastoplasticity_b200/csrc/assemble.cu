@@ -386,14 +386,14 @@ __global__ void __launch_bounds__(128) assemble_rows_reg_kernel(const AsmArgs A)
     }
 }
 
-// ---- variant C: TMA-staged (P1, node degree <= 8) ---------------------------------------------------
+// ---- TMA staging of the P1 kernel (variant D; node degree <= 8) -------------------------------------
 // The elements touched by the 32 nodes of a slice form (on structured meshes) two runs of consecutive ids, each covered
 // by one fixed-width box (plan: stage_box).  One lane brings the boxes into warp-private shared memory with 2-D TMA
 // tensor copies (cp.async.bulk.tensor.2d completing on an mbarrier): one copy per tensor and box - all 7 geometry rows,
 // all 9 DS rows, the 3 S rows - so 3 copies per box instead of 19 row copies (a 1-D bulk-copy version was TMA
 // issue-rate bound, ~50 cycles per copy per SM).  Each element is fetched once per slice, fully coalesced, with ~20 KB
 // in flight per warp regardless of occupancy; the accumulation then runs out of shared memory with exactly the
-// arithmetic of variants A/B.  Slices that need more than two boxes take the direct-load path of variant B.
+// arithmetic of variants A/B.  Slices that need more than two boxes take direct loads.
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 
 struct alignas(64) StageMaps {
@@ -425,161 +425,6 @@ __device__ __forceinline__ void tma_box_2d(uint32_t dst, const CUtensorMap* map,
                : "memory");
 }
 
-template <int MODE, bool FORCE, int MAXDEG>
-__global__ void __launch_bounds__(128) assemble_rows_tma_kernel(const AsmArgs A, const __grid_constant__ StageMaps M) {
-  constexpr int NP = 3;
-  using L = StageLayout<MODE, FORCE>;
-  extern __shared__ __align__(128) unsigned char smem_raw[];
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int64_t slice = (int64_t)blockIdx.x * (blockDim.x >> 5) + warp;
-  if (slice >= A.n_slices) return;  // warp-uniform; only warp-level synchronisation below
-  const int bw = A.boxw;
-  unsigned char* wbase = smem_raw + (size_t)warp * L::warp_b(bw);
-  uint64_t* mbar = reinterpret_cast<uint64_t*>(wbase + 2 * L::box_b(bw));
-  const int n_box = A.stage_box[slice * 3] & 0xFF;
-  const bool staged = n_box >= 1 && n_box <= 2;  // warp-uniform
-  if (staged) {
-    if (lane == 0) {
-      asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(mbar)), "r"(1));
-      asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncwarp();
-    if (lane == 0) {
-      const uint32_t bar = smem_u32(mbar);
-      const uint32_t bytes_per_box = (uint32_t)((7 + L::NRAW + (FORCE ? 3 : 0)) * bw * 8);
-      asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes_per_box * (uint32_t)n_box) : "memory");
-      for (int b = 0; b < n_box; ++b) {
-        const int start = A.stage_box[slice * 3 + 1 + b];
-        unsigned char* bb = wbase + (size_t)b * L::box_b(bw);
-        tma_box_2d(smem_u32(bb), &M.geom, start, bar);
-        bb += L::geom_b(bw);
-        tma_box_2d(smem_u32(bb), &M.t0, start, bar);
-        bb += L::t0_b(bw);
-        if (MODE == MODE_ELASTIC || MODE == MODE_TANGENT_REF) {
-          tma_box_2d(smem_u32(bb), &M.t1, start, bar);
-          bb += L::t1_b(bw);
-        }
-        if (MODE == MODE_TANGENT_REF) {
-          tma_box_2d(smem_u32(bb), &M.t2, start, bar);
-          bb += L::t2_b(bw);
-        }
-        if (FORCE) tma_box_2d(smem_u32(bb), &M.s, start, bar);
-      }
-    }
-  }
-  // while the copies fly: node bookkeeping, incidence words, accumulator init
-  const int64_t a = slice * 32 + lane;
-  int deg = 0;
-  int64_t base = 0;
-  if (a < A.n_n) {
-    const int nb = A.nbr_ptr[a];
-    deg = A.nbr_ptr[a + 1] - nb;
-    base = 4 * (int64_t)nb;
-  }
-  const int64_t sbase = A.slice_ptr[slice];
-  const int width = (int)((A.slice_ptr[slice + 1] - sbase) >> 5);
-  constexpr int CH = 8;  // plan guarantees width <= 8 when stage_ok
-  uint32_t words[CH];
-#pragma unroll
-  for (int i = 0; i < CH; ++i) words[i] = (i < width) ? __ldcs(A.inc_stage + sbase + (int64_t)i * 32 + lane) : 0u;
-  double acc[MAXDEG][4];
-#pragma unroll
-  for (int j = 0; j < MAXDEG; ++j) acc[j][0] = acc[j][1] = acc[j][2] = acc[j][3] = 0.0;
-  double f0 = 0.0, f1 = 0.0;
-  if (staged) {
-    const uint32_t bar = smem_u32(mbar);
-    uint32_t ok = 0;
-    do {
-      asm volatile("{ .reg .pred p; mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2; selp.u32 %0, 1, 0, p; }"
-                   : "=r"(ok)
-                   : "r"(bar), "r"(0)
-                   : "memory");
-    } while (!ok);
-  }
-#pragma unroll 1
-  for (int i = 0; i < width; ++i) {
-    const uint32_t word = words[0];
-#pragma unroll
-    for (int k = 0; k + 1 < CH; ++k) words[k] = words[k + 1];
-    if (!(word & 0x80000000u)) continue;
-    const int la = (word >> 9) & 3;
-    PointData<NP, MODE, FORCE> pd;
-    if (staged) {
-      const int li = word & 0x1FF;
-      const int b = li >= bw ? 1 : 0;
-      const int o = li - b * bw;
-      const unsigned char* bb = wbase + (size_t)b * L::box_b(bw);
-      const double* g = reinterpret_cast<const double*>(bb) + o;
-      pd.w = g[0];
-#pragma unroll
-      for (int p = 0; p < NP; ++p) {
-        pd.d1[p] = g[(1 + p) * bw];
-        pd.d2[p] = g[(4 + p) * bw];
-      }
-      bb += L::geom_b(bw);
-      const double* t0 = reinterpret_cast<const double*>(bb) + o;
-      if (MODE == MODE_ELASTIC) {
-        pd.raw[0] = t0[0];
-        pd.raw[1] = (reinterpret_cast<const double*>(bb + L::t0_b(bw)) + o)[0];
-      } else {
-#pragma unroll
-        for (int k = 0; k < 9; ++k) pd.raw[k] = t0[k * bw];
-        if (MODE == MODE_TANGENT_REF) {
-          pd.raw[MODE == MODE_TANGENT_REF ? 9 : 0] = (reinterpret_cast<const double*>(bb + L::t0_b(bw)) + o)[0];
-          pd.raw[MODE == MODE_TANGENT_REF ? 10 : 0] = (reinterpret_cast<const double*>(bb + L::t0_b(bw) + L::t1_b(bw)) + o)[0];
-        }
-      }
-      if (FORCE) {
-        const double* sp = reinterpret_cast<const double*>(bb + L::t0_b(bw) + L::t1_b(bw) + L::t2_b(bw)) + o;
-#pragma unroll
-        for (int k = 0; k < 3; ++k) pd.s[k] = sp[k * bw];
-      }
-    } else {  // direct loads (slices with more than two boxes)
-      const uint32_t key = A.inc_key[sbase + (int64_t)i * 32 + lane];
-      load_point<NP, MODE, FORCE>(A, (int64_t)(key >> 3), pd);
-    }
-    double tx[3], ty[3];
-    point_terms<NP, MODE, FORCE>(A, pd, la, tx, ty, f0, f1);
-#pragma unroll
-    for (int lb = 0; lb < NP; ++lb) {
-      const int slot = (word >> (11 + 4 * lb)) & 15;
-      const double b1 = pd.d1[lb], b2 = pd.d2[lb];
-      const double p00 = tx[0] * b1, p01 = tx[2] * b2, p10 = tx[1] * b2, p11 = tx[2] * b1;
-      const double p20 = ty[0] * b1, p21 = ty[2] * b2, p30 = ty[1] * b2, p31 = ty[2] * b1;
-#define FEM_UPD(J)                               \
-  case J:                                        \
-    if (J < MAXDEG) {                            \
-      acc[J < MAXDEG ? J : 0][0] = (acc[J < MAXDEG ? J : 0][0] + p00) + p01; \
-      acc[J < MAXDEG ? J : 0][1] = (acc[J < MAXDEG ? J : 0][1] + p10) + p11; \
-      acc[J < MAXDEG ? J : 0][2] = (acc[J < MAXDEG ? J : 0][2] + p20) + p21; \
-      acc[J < MAXDEG ? J : 0][3] = (acc[J < MAXDEG ? J : 0][3] + p30) + p31; \
-    }                                            \
-    break;
-      switch (slot) {
-        FEM_UPD(0) FEM_UPD(1) FEM_UPD(2) FEM_UPD(3) FEM_UPD(4) FEM_UPD(5) FEM_UPD(6) FEM_UPD(7)
-        default: break;
-      }
-#undef FEM_UPD
-    }
-  }
-  if (a >= A.n_n) return;
-  if (FORCE) reinterpret_cast<double2*>(A.F)[a] = make_double2(f0, f1);
-  double2* row0 = reinterpret_cast<double2*>(A.K_vals + base);
-  double2* row1 = row0 + deg;
-#pragma unroll
-  for (int j = 0; j < MAXDEG; ++j)
-    if (j < deg) {
-      double2 v0 = make_double2(acc[j][0], acc[j][1]), v1 = make_double2(acc[j][2], acc[j][3]);
-      if (MODE == MODE_TANGENT_REF) {  // csr_plus_csr: K_elast + correction
-        const double2 k0 = reinterpret_cast<const double2*>(A.Kel + base)[j];
-        const double2 k1 = reinterpret_cast<const double2*>(A.Kel + base)[deg + j];
-        v0.x = k0.x + v0.x; v0.y = k0.y + v0.y; v1.x = k1.x + v1.x; v1.y = k1.y + v1.y;
-      }
-      __stcs(row0 + j, v0);
-      __stcs(row1 + j, v1);
-    }
-}
-
 #ifndef FEM_ASM_CHUNK
 #define FEM_ASM_CHUNK 2  // consecutive slices per claim of the dynamic scheduler of variant D (measured: 1: see NC, 2: 0.922 ms, 4: 0.942, 8: 0.992, 16: 1.176)
 #endif
@@ -590,10 +435,10 @@ __global__ void __launch_bounds__(128) assemble_rows_tma_kernel(const AsmArgs A,
 #define FEM_ASM_UNROLL 2  // incidence steps per rotation of the register queue in variant D (1, 2, 4 or 8)
 #endif
 // ---- variant D: persistent, software-pipelined TMA staging ------------------------------------------------------
-// Same staging and arithmetic as variant C, but each warp walks many slices and keeps the TMA engine one half-slice
-// ahead: box 0 of slice s+1 is requested as soon as the incidences living in box 0 of slice s are consumed, box 1 of
-// s+1 after box 1 of s.  The dependent chain (box table -> TMA -> compute -> store) of a slice is thereby overlapped
-// with the computation of the previous one without any extra shared memory.
+// Each warp walks many slices and keeps the TMA engine one half-slice ahead: box 0 of slice s+1 is requested as soon as
+// the incidences living in box 0 of slice s are consumed, box 1 of s+1 after box 1 of s.  The dependent chain (box table
+// -> TMA -> compute -> store) of a slice is thereby overlapped with the computation of the previous one without any extra
+// shared memory.
 __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
   uint32_t ok = 0;
   do {
@@ -959,193 +804,6 @@ __global__ void __launch_bounds__(352) assemble_rows_tmap_kernel(const AsmArgs A
   }
 }
 
-// ---- variant E: persistent TMA staging with the row accumulators in warp-private shared memory ---------------------
-// Same staging, slice scheduling and arithmetic as variant D.  D keeps the 4*MAXDEG accumulators of a node in registers
-// and must route every contribution through a `switch` on the (data-dependent) slot; that costs ~160 registers
-// (10 warps/SM) and ~310 executed instructions per incidence.  Here the accumulators live in a warp-private array
-// ps[slot][half][lane] of double2 (conflict-free when the lanes agree on the slot, i.e. on structured meshes), so a
-// contribution is "load 2 x 16 B, 8 adds, store 2 x 16 B" at a computed address: no dispatch, ~70 registers, less
-// than half the instructions.  A thread still owns its node's rows and adds contributions in ascending element order
-// ((acc + p00) + p01 per entry), so the values are bit-identical to variants A-D; the first contribution is added to
-// a zeroed accumulator, which is exact.
-template <int MODE, bool FORCE, int MAXDEG, int BW>
-__global__ void __launch_bounds__(256) assemble_rows_ps_kernel(const AsmArgs A, const __grid_constant__ StageMaps M) {
-  constexpr int NP = 3;
-  using L = StageLayout<MODE, FORCE>;
-  extern __shared__ __align__(128) unsigned char smem_raw[];
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int bw = BW ? BW : A.boxw;
-  constexpr int PS_BYTES = MAXDEG * 2 * 32 * 16;
-  const int warp_bytes = L::warp_b(bw) + PS_BYTES;
-  unsigned char* wbase = smem_raw + (size_t)warp * warp_bytes;
-  unsigned char* box0 = wbase;
-  unsigned char* box1 = wbase + L::box_b(bw);
-  uint64_t* mbar = reinterpret_cast<uint64_t*>(wbase + 2 * L::box_b(bw));
-  double2* ps = reinterpret_cast<double2*>(wbase + L::warp_b(bw)) + lane;  // ps[(slot*2 + half)*32]
-  const uint32_t bar0 = smem_u32(mbar), bar1 = smem_u32(mbar + 1);
-  if (lane == 0) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar0), "r"(1));
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar1), "r"(1));
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-#pragma unroll
-  for (int j = 0; j < 2 * MAXDEG; ++j) ps[j * 32] = make_double2(0.0, 0.0);
-  __syncwarp();
-  const int64_t n_slices = A.n_slices;
-  auto claim = [&]() -> int64_t {
-    unsigned long long v = 0;
-    if (lane == 0) v = atomicAdd(A.slice_counter, 1ULL);
-    return (int64_t)__shfl_sync(0xffffffffu, v, 0);
-  };
-  int64_t slice = claim();
-  int64_t slice1 = claim();
-  uint32_t ph0 = 0, ph1 = 0;
-  constexpr int CH = 8;
-  struct Book { int nb, cn, st0, st1, deg, width; int64_t base, sbase; };
-  auto load_box = [&](int64_t s, Book& k) {
-    k.nb = 0; k.cn = 0; k.st0 = 0; k.st1 = 0;
-    if (s < n_slices) {
-      const int raw = A.stage_box[s * 3];  // boxes | canonical flag << 8
-      k.nb = raw & 0xFF; k.cn = (raw >> 8) & 1; k.st0 = A.stage_box[s * 3 + 1]; k.st1 = A.stage_box[s * 3 + 2];
-    }
-  };
-  auto load_node = [&](int64_t s, Book& k) {
-    k.deg = 0; k.base = 0;
-    const int64_t a = s * 32 + lane;
-    if (s < n_slices && a < A.n_n) {
-      const int nbp = A.nbr_ptr[a];
-      k.deg = A.nbr_ptr[a + 1] - nbp;
-      k.base = 4 * (int64_t)nbp;
-    }
-  };
-  auto load_sell = [&](int64_t s, Book& k) {
-    k.sbase = 0; k.width = 0;
-    if (s < n_slices) { k.sbase = A.slice_ptr[s]; k.width = (int)((A.slice_ptr[s + 1] - k.sbase) >> 5); }
-  };
-  Book cur, nxt;
-  uint32_t words[CH], nwords[CH];
-  load_box(slice, cur); load_node(slice, cur); load_sell(slice, cur);
-  load_sell(slice1, nxt);
-#pragma unroll
-  for (int i = 0; i < CH; ++i) words[i] = (i < cur.width) ? __ldcs(A.inc_stage + cur.sbase + (int64_t)i * 32 + lane) : 0u;
-  if (slice < n_slices && lane == 0 && cur.nb >= 1 && cur.nb <= 2) {
-    issue_box<MODE, FORCE>(M, box0, bw, cur.st0, bar0);
-    if (cur.nb == 2) issue_box<MODE, FORCE>(M, box1, bw, cur.st1, bar1);
-  }
-  while (slice < n_slices) {
-    const int64_t next = slice1;
-    const int64_t slice2 = claim();
-    load_box(next, nxt);
-    load_node(next, nxt);
-#pragma unroll
-    for (int i = 0; i < CH; ++i) nwords[i] = (i < nxt.width) ? __ldcs(A.inc_stage + nxt.sbase + (int64_t)i * 32 + lane) : 0u;
-    Book nn;
-    load_sell(slice2, nn);
-    const int nb = cur.nb;
-    const bool staged = nb >= 1 && nb <= 2;
-    const int64_t a = slice * 32 + lane;
-    double f0 = 0.0, f1 = 0.0;
-#pragma unroll 1
-    for (int pass = 0; pass < 2; ++pass) {
-      if (staged) {
-        if (pass == 0) { mbar_wait(bar0, ph0); ph0 ^= 1; }
-        else if (nb == 2) { mbar_wait(bar1, ph1); ph1 ^= 1; }
-      }
-      if (pass == 0 || (staged && nb == 2)) {
-#pragma unroll
-        for (int i = 0; i < CH; ++i) {  // unrolled: words[i] is a register, no queue rotation
-          const uint32_t word = words[i];
-          const int li = word & 0x1FF;
-          if ((word & 0x80000000u) && !(staged && ((li >= bw) != (pass == 1)))) {
-            const int la = (word >> 9) & 3;
-            PointData<NP, MODE, FORCE> pd;
-            if (staged) {
-              const int o = li - pass * bw;
-              const unsigned char* bb = pass ? box1 : box0;
-              const double* g = reinterpret_cast<const double*>(bb) + o;
-              pd.w = g[0];
-#pragma unroll
-              for (int p = 0; p < NP; ++p) {
-                pd.d1[p] = g[(1 + p) * bw];
-                pd.d2[p] = g[(4 + p) * bw];
-              }
-              bb += L::geom_b(bw);
-              const double* t0 = reinterpret_cast<const double*>(bb) + o;
-              if (MODE == MODE_ELASTIC) {
-                pd.raw[0] = t0[0];
-                pd.raw[1] = (reinterpret_cast<const double*>(bb + L::t0_b(bw)) + o)[0];
-              } else {
-#pragma unroll
-                for (int k = 0; k < 9; ++k) pd.raw[k] = t0[k * bw];
-                if (MODE == MODE_TANGENT_REF) {
-                  pd.raw[MODE == MODE_TANGENT_REF ? 9 : 0] = (reinterpret_cast<const double*>(bb + L::t0_b(bw)) + o)[0];
-                  pd.raw[MODE == MODE_TANGENT_REF ? 10 : 0] = (reinterpret_cast<const double*>(bb + L::t0_b(bw) + L::t1_b(bw)) + o)[0];
-                }
-              }
-              if (FORCE) {
-                const double* sp = reinterpret_cast<const double*>(bb + L::t0_b(bw) + L::t1_b(bw) + L::t2_b(bw)) + o;
-#pragma unroll
-                for (int k = 0; k < 3; ++k) pd.s[k] = sp[k * bw];
-              }
-            } else {  // direct loads (slices with more than two boxes)
-              const uint32_t key = A.inc_key[cur.sbase + (int64_t)i * 32 + lane];
-              load_point<NP, MODE, FORCE>(A, (int64_t)(key >> 3), pd);
-            }
-            double tx[3], ty[3];
-            point_terms<NP, MODE, FORCE>(A, pd, la, tx, ty, f0, f1);
-#pragma unroll
-            for (int lb = 0; lb < NP; ++lb) {
-              const int slot = (word >> (11 + 4 * lb)) & 15;
-              double2* r = ps + slot * 64;
-              const double b1 = pd.d1[lb], b2 = pd.d2[lb];
-              double2 v0 = r[0], v1 = r[32];
-              v0.x = (v0.x + tx[0] * b1) + tx[2] * b2;  // K[2a  , 2b  ]
-              v0.y = (v0.y + tx[1] * b2) + tx[2] * b1;  // K[2a  , 2b+1]
-              v1.x = (v1.x + ty[0] * b1) + ty[2] * b2;  // K[2a+1, 2b  ]
-              v1.y = (v1.y + ty[1] * b2) + ty[2] * b1;  // K[2a+1, 2b+1]
-              r[0] = v0;
-              r[32] = v1;
-            }
-          }
-        }
-      }
-      __syncwarp();  // every lane is done reading this pass's box: it may be overwritten by the next slice's copy
-      if (lane == 0 && nxt.nb >= 1 && nxt.nb <= 2) {
-        if (pass == 0) issue_box<MODE, FORCE>(M, box0, bw, nxt.st0, bar0);
-        else if (nxt.nb == 2) issue_box<MODE, FORCE>(M, box1, bw, nxt.st1, bar1);
-      }
-    }
-    {
-      const int deg = (a < A.n_n) ? cur.deg : 0;
-      if (FORCE && a < A.n_n) reinterpret_cast<double2*>(A.F)[a] = make_double2(f0, f1);
-      double2* row0 = reinterpret_cast<double2*>(A.K_vals + cur.base);
-      double2* row1 = row0 + deg;
-#pragma unroll
-      for (int j = 0; j < MAXDEG; ++j) {
-        if (j < deg) {
-          double2 v0 = ps[j * 64], v1 = ps[j * 64 + 32];
-          if (MODE == MODE_TANGENT_REF) {  // csr_plus_csr: K_elast + correction
-            const double2 k0 = reinterpret_cast<const double2*>(A.Kel + cur.base)[j];
-            const double2 k1 = reinterpret_cast<const double2*>(A.Kel + cur.base)[deg + j];
-            v0.x = k0.x + v0.x; v0.y = k0.y + v0.y; v1.x = k1.x + v1.x; v1.y = k1.y + v1.y;
-          }
-          __stcs(row0 + j, v0);
-          __stcs(row1 + j, v1);
-          ps[j * 64] = make_double2(0.0, 0.0);  // ready for the next slice
-          ps[j * 64 + 32] = make_double2(0.0, 0.0);
-        }
-      }
-    }
-    slice = next;
-    slice1 = slice2;
-    cur.nb = nxt.nb; cur.st0 = nxt.st0; cur.st1 = nxt.st1; cur.deg = nxt.deg; cur.base = nxt.base;
-    cur.sbase = nxt.sbase; cur.width = nxt.width;
-    nxt.sbase = nn.sbase; nxt.width = nn.width;
-#pragma unroll
-    for (int i = 0; i < CH; ++i) words[i] = nwords[i];
-  }
-}
-
 template <int MODE, bool FORCE>
 static int launch_assemble_tma(const fem_plan* P, AsmArgs& A, cudaStream_t st) {
   using L = StageLayout<MODE, FORCE>;
@@ -1171,45 +829,32 @@ static int launch_assemble_tma(const fem_plan* P, AsmArgs& A, cudaStream_t st) {
     }
   }
   if (FORCE && (rc = fem_encode_rows_map(&M.s, A.S, P->n_int, 3, bw)) != FEM_OK) return rc;
-  int warps = 4;
-  size_t smem = (size_t)warps * L::warp_b(bw);
-  if (smem > 227 * 1024) return -1;
-  if (g_fem_tuning.assemble_variant == 7) {  // one slice per warp (C); the default is D for every mode: 0.740 vs 0.831 ms for K_elast
-    auto kern = assemble_rows_tma_kernel<MODE, FORCE, 8>;
-    FEM_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    kern<<<(unsigned)fem_div_up(P->n_slices, warps), warps * 32, smem, st>>>(A, M);
-  } else {                                   // persistent, software-pipelined: D (register accumulators) or E (shared-memory accumulators)
-    const bool ps = g_fem_tuning.assemble_variant == 8;  // D unless E is asked for (E is shared-memory-bandwidth bound: profiles/r2c)
-    void (*kern)(const AsmArgs, const StageMaps) =
-        ps ? ((bw == 66) ? assemble_rows_ps_kernel<MODE, FORCE, 8, 66> : assemble_rows_ps_kernel<MODE, FORCE, 8, 0>)
-           : ((bw == 66) ? assemble_rows_tmap_kernel<MODE, FORCE, 8, 66> : assemble_rows_tmap_kernel<MODE, FORCE, 8, 0>);
-    const size_t per_warp = (size_t)L::warp_b(bw) + (ps ? 8 * 2 * 32 * 16 : 0);
-    // warps per CTA that packs the most warps into the 227 KB of an SM (1 KB per CTA is reserved)
-    int best = 0;
-    for (int w = (ps ? 1 : 4); w <= (ps ? 8 : 11); ++w) {
-      const size_t sm = (size_t)w * per_warp;
-      const int per = (int)((227 * 1024) / (sm + 1024));
-      if (per * w >= best) { best = per * w; warps = w; }
-    }
-    if (g_fem_tuning.assemble_warps >= 1 && g_fem_tuning.assemble_warps <= (ps ? 8 : 11)) warps = g_fem_tuning.assemble_warps;
-    smem = (size_t)warps * per_warp;
-    if (smem > 227 * 1024) return -1;
-    FEM_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    int per_sm = 0;
-    FEM_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, warps * 32, smem));
-    if (per_sm < 1) return -1;
-    int64_t blocks = (int64_t)per_sm * P->sm_count;
-    const int64_t need = fem_div_up(P->n_slices, warps);
-    if (blocks > need) blocks = need;
-    // one of FEM_SLICE_COUNTERS counters of this plan, round-robin per launch (atomic: host threads may launch concurrently),
-    // so up to FEM_SLICE_COUNTERS launches of one plan may be in flight on different streams without sharing a counter
-    // (variant D spreads its claims over FEM_ASM_NC interleaved counters: a group of FEM_ASM_NC consecutive ones)
-    static std::atomic<unsigned> launch_no{0};
-    static_assert(FEM_SLICE_COUNTERS % FEM_ASM_NC == 0, "counter groups");
-    A.slice_counter = reinterpret_cast<unsigned long long*>(P->dscratch + 8) + FEM_ASM_NC * (launch_no.fetch_add(1u) % (FEM_SLICE_COUNTERS / FEM_ASM_NC));
-    FEM_CUDA_CHECK(cudaMemsetAsync(A.slice_counter, 0, FEM_ASM_NC * sizeof(unsigned long long), st));
-    kern<<<(unsigned)blocks, warps * 32, smem, st>>>(A, M);
+  auto kern = (bw == 66) ? assemble_rows_tmap_kernel<MODE, FORCE, 8, 66> : assemble_rows_tmap_kernel<MODE, FORCE, 8, 0>;
+  const size_t per_warp = L::warp_b(bw);
+  // warps per CTA that packs the most warps into the 227 KB of an SM (1 KB per CTA is reserved)
+  int warps = 4, best = 0;
+  for (int w = 4; w <= 11; ++w) {
+    const size_t sm = (size_t)w * per_warp;
+    const int per = (int)((227 * 1024) / (sm + 1024));
+    if (per * w >= best) { best = per * w; warps = w; }
   }
+  const size_t smem = (size_t)warps * per_warp;
+  if (smem > 227 * 1024) return -1;
+  FEM_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  int per_sm = 0;
+  FEM_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, warps * 32, smem));
+  if (per_sm < 1) return -1;
+  int64_t blocks = (int64_t)per_sm * P->sm_count;
+  const int64_t need = fem_div_up(P->n_slices, warps);
+  if (blocks > need) blocks = need;
+  // one of FEM_SLICE_COUNTERS counters of this plan, round-robin per launch (atomic: host threads may launch concurrently),
+  // so up to FEM_SLICE_COUNTERS launches of one plan may be in flight on different streams without sharing a counter
+  // (the kernel spreads its claims over FEM_ASM_NC interleaved counters: a group of FEM_ASM_NC consecutive ones)
+  static std::atomic<unsigned> launch_no{0};
+  static_assert(FEM_SLICE_COUNTERS % FEM_ASM_NC == 0, "counter groups");
+  A.slice_counter = reinterpret_cast<unsigned long long*>(P->dscratch + 8) + FEM_ASM_NC * (launch_no.fetch_add(1u) % (FEM_SLICE_COUNTERS / FEM_ASM_NC));
+  FEM_CUDA_CHECK(cudaMemsetAsync(A.slice_counter, 0, FEM_ASM_NC * sizeof(unsigned long long), st));
+  kern<<<(unsigned)blocks, warps * 32, smem, st>>>(A, M);
   FEM_CUDA_CHECK(cudaGetLastError());
   return FEM_OK;
 }
@@ -1257,7 +902,7 @@ static int launch_assemble(const fem_plan* P, AsmArgs& A, cudaStream_t st) {
   // tangent (reads K_elast in its write-out) takes it where the straight-line path with 256-bit accesses covers most slices
   // (1.14 ms against 1.51 ms of the register kernel), else the register kernel
   const bool ref_tma = MODE != MODE_TANGENT_REF || (2 * P->stage_canon_slices >= P->n_slices && g_fem_tuning.assemble_canon != 2);
-  if (MODE != MODE_FORCE_ONLY && P->stage_ok && ((variant == 0 && ref_tma) || (variant == 6 || variant == 7 || variant == 8))) {
+  if (MODE != MODE_FORCE_ONLY && P->stage_ok && ((variant == 0 && ref_tma) || variant == 6)) {
     const int rc = launch_assemble_tma<MODE == MODE_FORCE_ONLY ? MODE_TANGENT : MODE, FORCE>(P, A, st);
     if (rc >= 0) return rc;  // -1: inputs not 16-byte aligned / too much shared memory -> register kernel
   }
@@ -1273,7 +918,7 @@ static int launch_assemble(const fem_plan* P, AsmArgs& A, cudaStream_t st) {
       return FEM_OK;
     }
   }
-  const int warps = (g_fem_tuning.assemble_warps >= 1 && g_fem_tuning.assemble_warps <= 4) ? g_fem_tuning.assemble_warps : 4;
+  const int warps = 4;
   int acc_rows = (MODE == MODE_FORCE_ONLY) ? 0 : 4 * P->max_degree;
   A.acc_rows = acc_rows;
   size_t smem = (size_t)warps * acc_rows * ACC_LD * sizeof(double);
@@ -1313,9 +958,9 @@ static void fill_args(const fem_plan* P, AsmArgs& A) {
   A.dphi1 = P->dphi1; A.dphi2 = P->dphi2; A.weight = P->weight;
   A.geom_rec = P->geom_rec; A.geom_rs = P->geom_rs;
   elastic_coeffs(A.dev2, A.vol);
-  // tuning key assemble_canon: 0 auto = regular-triangulation fast path with 256-bit row stores, 3 = fast path with the
-  // 16-byte stores of the generic path, 2 = fast path off
-  A.canon = g_fem_tuning.assemble_canon == 2 ? 0 : (g_fem_tuning.assemble_canon == 3 ? 2 : 1);
+  // tuning key assemble_canon: 0 auto = regular-triangulation fast path with 256-bit row stores (launch_assemble_tma drops to
+  // the 16-byte stores of the generic path when K is not 32-byte aligned), 2 = fast path off
+  A.canon = g_fem_tuning.assemble_canon == 2 ? 0 : 1;
 }
 
 extern "C" int fem_assemble_elastic(const fem_plan* P, const double* shear, const double* bulk, double* K_vals,
@@ -1407,63 +1052,6 @@ __global__ void __launch_bounds__(256) strain_kernel(int64_t n_e, const int32_t*
   }
 }
 
-// P1 (one integration point per element): the three gradients are recomputed from the node coordinates with the
-// operations of geometry_kernel (plan.cu) in the same order, so they are the stored values bit for bit - and the kernel
-// moves 12 B of node ids + two 16-byte gathers per node (served by L1/L2: a node is shared by six elements) instead of
-// streaming 48 B of stored gradients per element: compulsory traffic 12 + 8 + 8 + 24 B/element.  Measured at 16M elements:
-// 0.308 ms against 0.221 ms of the stored-gradient kernel - six more 16-byte gathers per element cost more in L2 than the
-// 48 streamed bytes cost in HBM - so it is NOT the default (tuning key strain_variant = 2 selects it; tested bit-identical).
-__global__ void __launch_bounds__(256) strain_p1_kernel(int64_t n_e, FemRefElem ref, const int32_t* __restrict__ elem,
-                                                        const double2* __restrict__ coord2, const double* __restrict__ u,
-                                                        double* __restrict__ E) {
-  for (int64_t g = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; g < n_e; g += (int64_t)gridDim.x * blockDim.x) {
-    int32_t nd[3];
-    int pp[3];
-    double a1[3], a2[3];
-    double j11 = 0.0, j12 = 0.0, j21 = 0.0, j22 = 0.0;
-#pragma unroll
-    for (int p = 0; p < 3; ++p) {
-      nd[p] = __ldcs(elem + (int64_t)p * n_e + g);
-      pp[p] = p;
-      const double2 c = __ldg(coord2 + nd[p]);
-      const double h1 = ref.dhat1[p], h2 = ref.dhat2[p];
-      j11 = j11 + c.x * h1;
-      j12 = j12 + c.y * h1;
-      j21 = j21 + c.x * h2;
-      j22 = j22 + c.y * h2;
-    }
-    const double det = j11 * j22 - j12 * j21;
-    const double i11 = j22 / det, i12 = -j12 / det, i21 = -j21 / det, i22 = j11 / det;
-#pragma unroll
-    for (int p = 0; p < 3; ++p) {
-      const double h1 = ref.dhat1[p], h2 = ref.dhat2[p];
-      a1[p] = i11 * h1 + i12 * h2;
-      a2[p] = i21 * h1 + i22 * h2;
-    }
-#pragma unroll
-    for (int i = 1; i < 3; ++i)  // ascending node id: csr_matvec order (see strain_kernel)
-#pragma unroll
-      for (int j = i; j > 0; --j)
-        if (nd[j - 1] > nd[j]) {
-          const int32_t tn = nd[j]; nd[j] = nd[j - 1]; nd[j - 1] = tn;
-          const int tp = pp[j]; pp[j] = pp[j - 1]; pp[j - 1] = tp;
-        }
-    double e0 = 0.0, e1 = 0.0, e2 = 0.0;
-#pragma unroll
-    for (int s = 0; s < 3; ++s) {
-      const double2 uv = __ldg(reinterpret_cast<const double2*>(u) + nd[s]);
-      const double b1 = pp[s] == 0 ? a1[0] : (pp[s] == 1 ? a1[1] : a1[2]);
-      const double b2 = pp[s] == 0 ? a2[0] : (pp[s] == 1 ? a2[1] : a2[2]);
-      e0 = e0 + b1 * uv.x;
-      e1 = e1 + b2 * uv.y;
-      e2 = (e2 + b2 * uv.x) + b1 * uv.y;
-    }
-    __stcs(E + g, e0);
-    __stcs(E + n_e + g, e1);
-    __stcs(E + 2 * n_e + g, e2);
-  }
-}
-
 extern "C" int fem_strain(const fem_plan* P, const double* u, double* E, fem_stream stream) {
   FEM_REQUIRE(P && u && E, "null pointer");
   FEM_REQUIRE((reinterpret_cast<uintptr_t>(u) & 15u) == 0, "u must be 16-byte aligned");
@@ -1473,10 +1061,8 @@ extern "C" int fem_strain(const fem_plan* P, const double* u, double* E, fem_str
   const unsigned blocks = (unsigned)b;
   cudaStream_t st = (cudaStream_t)stream;
 #define STRAIN(NP, NQ) strain_kernel<NP, NQ><<<blocks, threads, 0, st>>>(P->n_e, P->elem, P->dphi1, P->dphi2, u, E)
-  if (P->n_p == 3 && P->n_q == 1) {
-    if (P->coord2 && g_fem_tuning.strain_variant == 2) strain_p1_kernel<<<blocks, threads, 0, st>>>(P->n_e, P->ref, P->elem, P->coord2, u, E);
-    else STRAIN(3, 1);
-  } else if (P->n_p == 6 && P->n_q == 7) STRAIN(6, 7);
+  if (P->n_p == 3 && P->n_q == 1) STRAIN(3, 1);
+  else if (P->n_p == 6 && P->n_q == 7) STRAIN(6, 7);
   else if (P->n_p == 4 && P->n_q == 4) STRAIN(4, 4);
   else if (P->n_p == 8 && P->n_q == 9) STRAIN(8, 9);
   else {

@@ -27,16 +27,13 @@ int fem_encode_rows_map(CUtensorMap* out, const double* base, int64_t n_int, int
 void fem_set_error(const char* fmt, ...);
 
 struct FemTuning {
-  int return_map_variant;  // 0 auto, 1 scalar/256, 2 double2/128, 3 double2/256
-  int assemble_warps;      // warps per block of the assembly kernel (0 = 4)
   int spmv_group;          // lanes per node in the SpMV (0 = by degree)
   int spmv_blocks_per_sm;  // 0 = 32
-  int assemble_variant;    // 0 auto, 1 shared-memory accumulators (A), 2 register accumulators (B), 7 one-shot TMA (C), 6 persistent TMA (D), 8 persistent TMA with shared-memory accumulators (E)
+  int assemble_variant;    // 0 auto, 1 shared-memory accumulators (A), 2 register accumulators (B), 6 persistent TMA (D)
   int spmv_unroll;         // nodes per lane group in flight (0 = default)
   int spmv_staged;         // 0 auto (every operand streamed through shared memory when the tiles fit, else as 2), 1 gather x from global memory (round-1 kernel), 2 x staged, matrix through registers
   int peer_timeout_ms;     // bound of the in-kernel waits of the fused multi-GPU PCG (0 = 10 000 ms)
   int assemble_canon;      // 0 auto (straight-line path for slices of the reference's regular triangulation), 2 off
-  int strain_variant;      // 0/1 stored gradients (default), 2 P1 gradients recomputed from the coordinates (slower: L2 gathers)
   int mg_stencil_sym;      // 0 auto: coarse-level stencil sweeps read the lower half of the (symmetric) stencil as transposes of the neighbours' upper half; 2 = read all 36 planes
   int mg_fine_lattice;     // 0 auto: the V-cycle's level-0 smoother and residual read the lattice stencil when the descriptor carries one; 2 = the block-CSR copy
   int peer_nowait;         // DIAGNOSTIC ONLY: fused multi-GPU PCG kernels skip their waits (wrong results; isolates the wait time)
@@ -90,7 +87,6 @@ struct fem_plan {
   double* dphi1;   // [n_p][n_int]
   double* dphi2;   // [n_p][n_int]
   double* weight;  // [n_int]
-  double2* coord2;  // [n_n] node coordinates (x, y) interleaved: one 16-byte gather per node (P1 strain kernel)
   // scratch
   double* dscratch;  // small device scratch: 8 doubles (PCG scalars) + FEM_SLICE_COUNTERS 8-byte counters
   double* red_partials;  // [3][FEM_RED_MAXB] block sums + ticket counter of the order-deterministic dot products of this plan's SpMV

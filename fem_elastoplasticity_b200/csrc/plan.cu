@@ -22,18 +22,19 @@ extern "C" int fem_version(void) { return 100; }
 FemTuning g_fem_tuning = {};
 extern "C" int fem_set_tuning(const char* key, int value) {
   FEM_REQUIRE(key != nullptr, "key");
-  if (!strcmp(key, "return_map_variant")) g_fem_tuning.return_map_variant = value;
-  else if (!strcmp(key, "assemble_warps")) g_fem_tuning.assemble_warps = value;
-  else if (!strcmp(key, "spmv_group")) g_fem_tuning.spmv_group = value;
+  if (!strcmp(key, "spmv_group")) g_fem_tuning.spmv_group = value;
   else if (!strcmp(key, "spmv_blocks_per_sm")) g_fem_tuning.spmv_blocks_per_sm = value;
-  else if (!strcmp(key, "assemble_variant")) g_fem_tuning.assemble_variant = value;
-  else if (!strcmp(key, "spmv_unroll")) g_fem_tuning.spmv_unroll = value;
+  else if (!strcmp(key, "assemble_variant")) {
+    FEM_REQUIRE(value == 0 || value == 1 || value == 2 || value == 6, "assemble_variant is 0, 1, 2 or 6");
+    g_fem_tuning.assemble_variant = value;
+  } else if (!strcmp(key, "spmv_unroll")) g_fem_tuning.spmv_unroll = value;
   else if (!strcmp(key, "spmv_staged")) g_fem_tuning.spmv_staged = value;
   else if (!strcmp(key, "peer_timeout_ms")) g_fem_tuning.peer_timeout_ms = value;
   else if (!strcmp(key, "peer_nowait")) g_fem_tuning.peer_nowait = value;
-  else if (!strcmp(key, "strain_variant")) g_fem_tuning.strain_variant = value;
-  else if (!strcmp(key, "assemble_canon")) g_fem_tuning.assemble_canon = value;
-  else if (!strcmp(key, "mg_stencil_sym")) g_fem_tuning.mg_stencil_sym = value;
+  else if (!strcmp(key, "assemble_canon")) {
+    FEM_REQUIRE(value == 0 || value == 2, "assemble_canon is 0 or 2");
+    g_fem_tuning.assemble_canon = value;
+  } else if (!strcmp(key, "mg_stencil_sym")) g_fem_tuning.mg_stencil_sym = value;
   else if (!strcmp(key, "mg_fine_lattice")) g_fem_tuning.mg_fine_lattice = value;
   else {
     fem_set_error("unknown tuning key %s", key);
@@ -699,11 +700,6 @@ __global__ void build_geom_records(int64_t n_int, int n_p, int rs, const double*
   }
 }
 
-__global__ void interleave_coord(int64_t n_n, const double* __restrict__ coord, double2* __restrict__ out) {
-  for (int64_t a = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; a < n_n; a += (int64_t)gridDim.x * blockDim.x)
-    out[a] = make_double2(coord[a], coord[n_n + a]);
-}
-
 static int launch_geometry(fem_plan* P, const double* coord, int* d_bad, cudaStream_t st) {
   const int threads = 256;
   const unsigned blocks = (unsigned)fem_div_up(P->n_int, threads);
@@ -827,8 +823,6 @@ static int build_plan(fem_plan* P, const int32_t* elem, const double* coord, cud
     P->red_ticket = reinterpret_cast<unsigned*>(P->red_partials + 3 * FEM_RED_MAXB);
     cudaMemsetAsync(P->red_ticket, 0, 8 * sizeof(double), st);
     if ((rc = launch_geometry(P, coord, flags + 3, st)) != FEM_OK) break;
-    if ((rc = dmalloc(P, &P->coord2, n_n)) != FEM_OK) break;
-    interleave_coord<<<grid(n_n), threads, 0, st>>>(n_n, coord, P->coord2);
     // TMA staging plan (P1 meshes of bounded valence whose slices touch few runs of consecutive elements)
     P->stage_ok = 0;
     if (n_p == 3 && P->n_q == 1 && P->max_degree <= 8 && P->max_inc <= 8 && (P->n_int % 2) == 0 && P->n_int >= 64) {
@@ -930,7 +924,7 @@ extern "C" int fem_plan_destroy(fem_plan* P) {
   cudaFree(P->stage_box); cudaFree(P->inc_stage); cudaFree(P->tile_seg); cudaFree(P->nbr_loc);
   cudaFree(P->elem); cudaFree(P->nbr_ptr); cudaFree(P->nbr_idx); cudaFree(P->row_ptr); cudaFree(P->col_idx);
   cudaFree(P->inc_cnt); cudaFree(P->slice_ptr); cudaFree(P->inc_key); cudaFree(P->inc_meta);
-  cudaFree(P->geom); cudaFree(P->dscratch); cudaFree(P->coord2); cudaFree(P->geom_rec); cudaFree(P->red_partials);
+  cudaFree(P->geom); cudaFree(P->dscratch); cudaFree(P->geom_rec); cudaFree(P->red_partials);
   delete P;
   return FEM_OK;
 }

@@ -1,4 +1,4 @@
-// K5: Drucker-Prager return mapping + consistent tangent, one thread per pair of Gauss points.
+// K5: Drucker-Prager return mapping + consistent tangent, one thread per Gauss point.
 // Follows construct_constitutive_problem (Plasticity2D_DP/pythonFEM.py:604-757,
 // tsx-tunnel/pythonFEM.py:990-1157) operation by operation; compiled with -fmad=false.
 // Pure streaming: 193 B/point (+40 B when the plastic strain / multiplier are written).
@@ -84,85 +84,48 @@ __device__ __forceinline__ void dp_point(const DpConst& k, double e0, double e1,
   }
 }
 
-template <int V> struct Vec;
-template <> struct Vec<1> {
-  using T = double;
-  static __device__ __forceinline__ double get(const T& v, int) { return v; }
-  static __device__ __forceinline__ void set(T& v, int, double x) { v = x; }
-};
-template <> struct Vec<2> {
-  using T = double2;
-  static __device__ __forceinline__ double get(const T& v, int i) { return i ? v.y : v.x; }
-  static __device__ __forceinline__ void set(T& v, int i, double x) { if (i) v.y = x; else v.x = x; }
-};
-
-template <int V, int THREADS, int MINB>
-__global__ void __launch_bounds__(THREADS, MINB) dp_return_map_kernel(
-    int64_t n_vec, int64_t n_int, DpConst k, const double* __restrict__ E, double* Ep_prev,
+// One thread per Gauss point, 128 threads, 6 blocks per SM: measured best at 16M points (tools/tune.py) against two points
+// per thread (double2 loads and stores) and other block shapes.
+__global__ void __launch_bounds__(128, 6) dp_return_map_kernel(
+    int64_t n_int, DpConst k, const double* __restrict__ E, double* Ep_prev,
     const double* __restrict__ shear, const double* __restrict__ bulk, const double* __restrict__ eta,
     const double* __restrict__ c, int apply, double* __restrict__ S, double* __restrict__ DS,
     uint8_t* __restrict__ ind_p, double* __restrict__ lambda, double* Ep_out, unsigned long long* counts) {
-  using VT = typename Vec<V>::T;
   __shared__ unsigned int s_cnt[2];
   if (threadIdx.x < 2) s_cnt[threadIdx.x] = 0;
   __syncthreads();
   unsigned int my_s = 0, my_a = 0;
-  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n_vec; i += (int64_t)gridDim.x * blockDim.x) {
-    auto ldv = [&](const double* base, int row) { return __ldcs(reinterpret_cast<const VT*>(base + row * n_int) + i); };
-    VT e0 = ldv(E, 0), e1 = ldv(E, 1), e2 = ldv(E, 2);
-    VT g = ldv(shear, 0), kb = ldv(bulk, 0), et = ldv(eta, 0), cc = ldv(c, 0);
-    VT p0, p1, p2, p3;
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n_int; i += (int64_t)gridDim.x * blockDim.x) {
+    auto ldv = [&](const double* base, int row) { return __ldcs(base + row * n_int + i); };
+    const double e0 = ldv(E, 0), e1 = ldv(E, 1), e2 = ldv(E, 2);
+    const double g = ldv(shear, 0), kb = ldv(bulk, 0), et = ldv(eta, 0), cc = ldv(c, 0);
+    double p0 = 0.0, p1 = 0.0, p2 = 0.0, p3 = 0.0;
     if (Ep_prev) {
       p0 = ldv(Ep_prev, 0); p1 = ldv(Ep_prev, 1); p2 = ldv(Ep_prev, 2); p3 = ldv(Ep_prev, 3);
-    } else {
-#pragma unroll
-      for (int j = 0; j < V; ++j) { Vec<V>::set(p0, j, 0.0); Vec<V>::set(p1, j, 0.0); Vec<V>::set(p2, j, 0.0); Vec<V>::set(p3, j, 0.0); }
     }
-    VT so[4], dso[9], epo[4], lo;
-    unsigned int fl[V];
-    bool any_plastic = false;
+    DpPoint o;
+    dp_point(k, e0, e1, e2, p0, p1, p2, p3, g, kb, et, cc, o);
+    my_s += (o.flag == 1);
+    my_a += (o.flag == 2);
+    auto stv = [&](double* base, int row, double v) { __stcs(base + row * n_int + i, v); };
 #pragma unroll
-    for (int j = 0; j < V; ++j) {
-      DpPoint o;
-      dp_point(k, Vec<V>::get(e0, j), Vec<V>::get(e1, j), Vec<V>::get(e2, j), Vec<V>::get(p0, j), Vec<V>::get(p1, j),
-               Vec<V>::get(p2, j), Vec<V>::get(p3, j), Vec<V>::get(g, j), Vec<V>::get(kb, j), Vec<V>::get(et, j),
-               Vec<V>::get(cc, j), o);
+    for (int q = 0; q < 4; ++q) stv(S, q, o.s[q]);
 #pragma unroll
-      for (int q = 0; q < 4; ++q) { Vec<V>::set(so[q], j, o.s[q]); Vec<V>::set(epo[q], j, o.ep[q]); }
-#pragma unroll
-      for (int q = 0; q < 9; ++q) Vec<V>::set(dso[q], j, o.ds[q]);
-      Vec<V>::set(lo, j, o.lam);
-      fl[j] = o.flag;
-      my_s += (o.flag == 1);
-      my_a += (o.flag == 2);
-      any_plastic |= (o.flag != 0);
-    }
-    auto stv = [&](double* base, int row, const VT& v) { __stcs(reinterpret_cast<VT*>(base + row * n_int) + i, v); };
-#pragma unroll
-    for (int q = 0; q < 4; ++q) stv(S, q, so[q]);
-#pragma unroll
-    for (int q = 0; q < 9; ++q) stv(DS, q, dso[q]);
-    if (V == 2) {
-      reinterpret_cast<uchar2*>(ind_p)[i] = make_uchar2(fl[0] != 0, fl[V - 1] != 0);
-    } else {
-      ind_p[i] = fl[0] != 0;
-    }
-    if (lambda) stv(lambda, 0, lo);
+    for (int q = 0; q < 9; ++q) stv(DS, q, o.ds[q]);
+    ind_p[i] = o.flag != 0;
+    if (lambda) stv(lambda, 0, o.lam);
     if (apply) {
-      if (Ep_prev && any_plastic) {  // in-place history update (ep aliases ep_prev, :751)
+      if (Ep_prev && o.flag != 0) {  // in-place history update (ep aliases ep_prev, :751)
 #pragma unroll
-        for (int q = 0; q < 4; ++q) reinterpret_cast<VT*>(Ep_prev + q * n_int)[i] = epo[q];
+        for (int q = 0; q < 4; ++q) Ep_prev[q * n_int + i] = o.ep[q];
       }
       if (Ep_out && Ep_out != Ep_prev) {
 #pragma unroll
-        for (int q = 0; q < 4; ++q) stv(Ep_out, q, epo[q]);
+        for (int q = 0; q < 4; ++q) stv(Ep_out, q, o.ep[q]);
       }
     } else if (Ep_out) {
-      VT z;
 #pragma unroll
-      for (int j = 0; j < V; ++j) Vec<V>::set(z, j, 0.0);
-#pragma unroll
-      for (int q = 0; q < 4; ++q) stv(Ep_out, q, z);
+      for (int q = 0; q < 4; ++q) stv(Ep_out, q, 0.0);
     }
   }
   if (counts) {
@@ -195,30 +158,11 @@ extern "C" int fem_dp_return_map(int64_t n_int, const double* E, const double* h
   int dev = 0, sms = 148;
   cudaGetDevice(&dev);
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-  cudaStream_t st = (cudaStream_t)stream;
-  auto aligned16 = [](const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; };
-  const bool vec2 = (n_int % 2 == 0) && aligned16(E) && aligned16(shear) && aligned16(bulk) && aligned16(eta) &&
-                    aligned16(c) && aligned16(S) && aligned16(DS) && aligned16(Ep_prev) && aligned16(lambda) &&
-                    aligned16(Ep_out) && ((reinterpret_cast<uintptr_t>(ind_p) & 1u) == 0);
-  int variant = g_fem_tuning.return_map_variant;
-  if (variant < 1 || variant > 6) variant = 5;  // measured best at 16M points (tools/tune.py): 1 point/thread, 128 threads, 6 blocks/SM
-  if (!vec2 && variant != 4 && variant != 5) variant = 1;
-  unsigned long long* cnt = reinterpret_cast<unsigned long long*>(counts);
   const int64_t cap = (int64_t)sms * 8 * 64;  // grid-stride beyond that
-#define RM_LAUNCH(V, T, MB, N)                                                                                     \
-  do {                                                                                                             \
-    int64_t blocks = ((N) + (T)-1) / (T);                                                                          \
-    if (blocks > cap) blocks = cap;                                                                                \
-    dp_return_map_kernel<V, T, MB><<<(unsigned)blocks, T, 0, st>>>(N, n_int, k, E, Ep_prev, shear, bulk, eta, c, apply, S, \
-                                                                   DS, ind_p, lambda, Ep_out, cnt);               \
-  } while (0)
-  if (variant == 1) RM_LAUNCH(1, 256, 2, n_int);
-  else if (variant == 2) RM_LAUNCH(2, 128, 3, n_int / 2);
-  else if (variant == 3) RM_LAUNCH(2, 256, 1, n_int / 2);
-  else if (variant == 4) RM_LAUNCH(1, 128, 4, n_int);
-  else if (variant == 5) RM_LAUNCH(1, 128, 6, n_int);
-  else RM_LAUNCH(2, 64, 6, n_int / 2);
-#undef RM_LAUNCH
+  int64_t blocks = (n_int + 127) / 128;
+  if (blocks > cap) blocks = cap;
+  dp_return_map_kernel<<<(unsigned)blocks, 128, 0, (cudaStream_t)stream>>>(n_int, k, E, Ep_prev, shear, bulk, eta, c, apply, S, DS, ind_p,
+                                                                           lambda, Ep_out, reinterpret_cast<unsigned long long*>(counts));
   FEM_CUDA_CHECK(cudaGetLastError());
   return FEM_OK;
 }

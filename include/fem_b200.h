@@ -348,10 +348,12 @@ int fem_midpoints_p2_fill(void* handle, const double* coord, double* coord_mid, 
                           int32_t* surf, fem_stream stream);
 int fem_midpoints_p2_destroy(void* handle, fem_stream stream);
 
-/* launch-shape knobs for benchmarking ("return_map_variant", "assemble_variant", "assemble_warps", "spmv_group", "spmv_blocks_per_sm",
- * "spmv_staged", "peer_timeout_ms", "strain_variant", "assemble_canon", "mg_stencil_sym", "mg_fine_lattice" (2: the V-cycle's
- * level 0 reads the block-CSR copy even when the descriptor carries the lattice stencil));
- * value 0 restores the default.  Results never depend on them.                                     */
+/* launch-shape knobs for benchmarking ("assemble_variant" (1: shared-memory accumulators, 2: register accumulators,
+ * 6: TMA-staged P1 kernel), "assemble_canon" (2: no straight-line path for the regular triangulation), "spmv_group",
+ * "spmv_blocks_per_sm", "spmv_unroll", "spmv_staged", "peer_timeout_ms", "mg_stencil_sym", "mg_fine_lattice" (2: the
+ * V-cycle's level 0 reads the block-CSR copy even when the descriptor carries the lattice stencil)); value 0 restores the
+ * default.  "assemble_variant" and "assemble_canon" return FEM_ERR_INVALID_ARG for a value not listed here.  Results never
+ * depend on them.                                                                                                     */
 int fem_set_tuning(const char* key, int value);
 
 #ifdef __cplusplus

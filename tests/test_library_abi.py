@@ -28,6 +28,27 @@ def test_library_exports_every_header_symbol():
     assert lib.fem_version() >= 100
 
 
+def test_set_tuning_rejects_removed_kernel_selections():
+    """Keys and values that selected deleted assembly, strain and return-map kernels fail loudly instead of silently timing
+    the default kernel; the kept assembly variants are still accepted."""
+    from fem_elastoplasticity_b200 import _lib
+    if not os.path.isfile(_lib.LIB_PATH):
+        import __graft_entry__
+        __graft_entry__.build()
+    lib = _lib.load()
+    try:
+        for key, value in ((b"assemble_variant", 7), (b"assemble_variant", 8), (b"assemble_canon", 3), (b"assemble_warps", 4),
+                           (b"strain_variant", 2), (b"return_map_variant", 1)):
+            assert lib.fem_set_tuning(key, value) != 0, (key, value)
+        for value in (0, 1, 2, 6):
+            assert lib.fem_set_tuning(b"assemble_variant", value) == 0, value
+        for value in (0, 2):
+            assert lib.fem_set_tuning(b"assemble_canon", value) == 0, value
+    finally:
+        assert lib.fem_set_tuning(b"assemble_variant", 0) == 0
+        assert lib.fem_set_tuning(b"assemble_canon", 0) == 0
+
+
 def test_no_cpu_fallback_without_device():
     """Without a CUDA device the product path must fail loudly (never fall back to the oracle / CPU)."""
     import torch

@@ -45,14 +45,11 @@ def main():
     out = {"n_e": P.n_e, "nnz": P.nnz, "n_dof": P.n_dof, "max_degree": P.max_degree, "stage": P.stage_info()}
     rm = {}
     res = {}
-    for v in (1, 2, 3, 4, 5, 6):
-        knob("return_map_variant", v)
-        res[f"return_map_v{v}_ms"] = timeit(lambda: dp_return_map(Es, ep, G, Kb, eta, c, want_ep=False, want_counts=True, out=rm))
-    knob("return_map_variant", 0)
+    res["return_map_ms"] = timeit(lambda: dp_return_map(Es, ep, G, Kb, eta, c, want_ep=False, want_counts=True, out=rm))
     r = dp_return_map(Es, ep, G, Kb, eta, c, want_ep=False, out=rm)
     kel_ref = None
     k, F = P.empty(P.nnz), P.empty(P.n_dof)
-    for v, name in ((2, "reg"), (7, "tma"), (6, "tmapipe"), (8, "ps"), (0, "default")):
+    for v, name in ((2, "reg"), (6, "tmapipe"), (0, "default")):
         knob("assemble_variant", v)
         res[f"assemble_elastic_{name}_ms"] = timeit(lambda: P.assemble_elastic(G, Kb, out=k))
         kel = k.clone()
@@ -64,11 +61,6 @@ def main():
             kel_ref, kt_ref, F_ref = kel, kt, F.clone()
         else:
             res[f"{name}_equals_reg_bits"] = bool(torch.equal(kel, kel_ref) and torch.equal(kt, kt_ref) and torch.equal(F, F_ref))
-    for w in (1, 2, 3, 4, 8):                        # warps per CTA of the persistent shared-memory-accumulator kernel (E)
-        knob("assemble_variant", 8), knob("assemble_warps", w)
-        res[f"assemble_tangent_force_ps_w{w}_ms"] = timeit(lambda: P.assemble_tangent_force(r["ds"], r["s"], out_k=k, out_f=F))
-        res[f"assemble_elastic_ps_w{w}_ms"] = timeit(lambda: P.assemble_elastic(G, Kb, out=k))
-    knob("assemble_warps", 0)
     knob("assemble_variant", 0)
     res["internal_force_ms"] = timeit(lambda: P.internal_force(r["s"], out=F))
     u = torch.randn(P.n_dof, dtype=torch.float64, device="cuda")
@@ -90,10 +82,6 @@ def main():
             else:
                 res[f"spmv_{name}_b{bps}_maxdiff"] = float((y - y_ref).abs().max() / y_ref.abs().max())
     knob("spmv_staged", 0), knob("spmv_blocks_per_sm", 0)
-    for w in (4, 5, 6, 8, 10, 11):                       # warps per CTA of the persistent register-accumulator kernel (D)
-        knob("assemble_variant", 6), knob("assemble_warps", w)
-        res[f"assemble_tangent_force_tmapipe_w{w}_ms"] = timeit(lambda: P.assemble_tangent_force(r["ds"], r["s"], out_k=k, out_f=F))
-    knob("assemble_warps", 0), knob("assemble_variant", 0)
     out["results"] = res
     print(json.dumps(out, indent=1))
 
